@@ -2,7 +2,7 @@
 """bench.py — one "step" = one pass of the CTR hot path (gather → attention → MLP → BCE → backward →
 scatter-add + SGD(rows) + Adam(dense)) over one batch of synthetic MovieLens-shaped input.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 Prints ONE JSON line (see the task contract).  `value` = whole-job train samples/s with inputs
 resident in HBM; `e2e` = same metric through the C-ABI entry point ctr_train_step_idx with pinned
@@ -120,6 +120,30 @@ def algorithmic_bytes(w, hist, ir):
     return gather, scatter, rows
 
 
+def dump_rows(batch, nrows=32768, seed=0):
+    """A fixed, seeded sample of `nrows` ITEM_EMB rows among those the batch updates (the whole table is up to 25.6 GB),
+    in ascending order."""
+    ur, ir, hist, y = batch
+    rows = np.unique(np.concatenate([hist[hist >= 0], ir[ir >= 0]]))
+    return np.sort(np.random.default_rng(seed).choice(rows, min(nrows, rows.size), replace=False))
+
+
+def step_outputs(eng, w, rows):
+    """What a caller of the timed step receives from its last call: the batch cost and the model the step leaves behind,
+    i.e. the dense weights in full and the ITEM_EMB rows `rows` (dump_rows of the step's batch).  The rows are read back
+    through the gather entry point, S rows per history slot; it gathers locally, so the table must not be row-sharded."""
+    S, D, uP = w["S"], w["D"], w["uP"]
+    slots = np.concatenate([rows, np.full(-rows.size % S, -1)]).astype(np.int32).reshape(-1, S)
+    none = np.full(slots.shape[0], -1, np.int32)
+    X = eng.gather_rows(none, none, slots)
+    out = {"cost": np.array([eng.last_cost()], np.float32)}
+    out.update(zip(("mlp0", "mlp1", "mlp2", "att0"), eng.get_weights()))
+    if w["model"] != "din":
+        del out["att0"]                  # the YouTube graph has no attention weights
+    out["item_emb_rows"] = X[:, uP:uP + S * D].reshape(-1, D)[:rows.size]
+    return out
+
+
 def config_of(args, w, wname, world):
     """identical keys for both arms (the driver compares them)"""
     return {"workload": wname, "note": w["note"], "graph": w["model"], "users": w["U"], "items": w["I"], "D": w["D"], "S": w["S"],
@@ -202,7 +226,7 @@ def run_reference(args, w, wname):
     emb = (rng.standard_normal((I, w["D"]), dtype=np.float32) / np.sqrt(w["D"])).astype(np.float32)
     tr = orc.IdxTrainer(ocfg, orc.default_solver(0), orc.init_weights(ocfg, 0), uf, itf, emb)
     batches = [make_batch(rng, w["U"], I, Bc, w["S"], zipf=w["zipf"]) for _ in range(2)]
-    steps = max(1, min(args.steps, 20)); warm = max(1, min(args.warmup, 2))
+    steps = args.steps; warm = max(1, min(args.warmup, 2))
 
     def one(th):
         t = time.perf_counter(); tr.step_fast(*batches[0], table_lr=0.05, nthreads=th); return time.perf_counter() - t
@@ -341,7 +365,13 @@ def main():
     ap.add_argument("--gemm", default="auto", choices=["auto", "fp32", "tcgen05"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-legs", action="store_true", help="only the timed workload (+ roofline, e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (cost, dense weights, a seeded "
+                    "sample of the updated ITEM_EMB rows) as DIR/<name>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "item2vec"):
+        ap.error("--dump-outputs covers the engine's CTR training step (--impl ours, not item2vec)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wname = args.workload
     if wname == "item2vec":
@@ -349,6 +379,10 @@ def main():
     w = dict(WORKLOADS[wname])
     if args.batch:
         w["B"] = args.batch
+    sharded = args.gpus > 1 and w["I"] * w["D"] * 4 > 32 * 2**20         # the engine row-shards ITEM_* tables above 32 MiB
+    if args.dump_outputs and sharded:
+        ap.error("--dump-outputs reads rows back through a local gather, which a row-sharded item table "
+                 "(%s on %d GPUs) does not serve" % (wname, args.gpus))
     if args.impl == "reference":
         return run_reference(args, w, wname)
 
@@ -400,8 +434,10 @@ def main():
 
     flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device=dev)      # > 126 MB L2
 
-    def timed_leg(eng, w, B, steps, warmup, profile=False, clocks=True, zipf=None, seed=100):
-        """K timed steps, inputs resident in HBM, L2 flushed before every step (outside the events)."""
+    def timed_leg(eng, w, B, steps, warmup, profile=False, clocks=True, zipf=None, seed=100, capture=False):
+        """K timed steps, inputs resident in HBM, L2 flushed before every step (outside the events).  capture: also
+        return step_outputs() of the last timed step, read back after the launch count and before the untimed tail
+        trains on; its rows are sampled before the clock sampler starts."""
         host = make_batches(w, B, 4, seed, zipf)
         devb = [tuple(torch.from_numpy(a).to(dev) for a in b) for b in host]
         st = torch.cuda.ExternalStream(eng.stream, device=dev)
@@ -414,6 +450,7 @@ def main():
                 if e: e[0].record(st)
                 eng.train_step_idx_dev(ur.data_ptr(), ir.data_ptr(), hist.data_ptr(), y.data_ptr(), B)
                 if e: e[1].record(st)
+        rows = dump_rows(host[(warmup + steps - 1) % len(host)]) if capture else None
         sampler = ClockSampler(local) if (clocks and not profile) else None      # polls from before the warm-up
         for i in range(warmup):
             one(i)
@@ -433,6 +470,7 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
         l2 = eng.launch_count()
+        outputs = step_outputs(eng, w, rows) if capture else None
         clk = None
         if sampler:      # untimed tail: the same steps keep the load up until nvidia-smi has had >= 0.3 s to sample it
             k = 0
@@ -452,7 +490,8 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
         cost = eng.last_cost()
-        return dict(ms=ms, wall=wall, clocks=clk, launches=(l2 - l1), host=host, cost=cost, prof=eng.profile_dump() if profile else None)
+        return dict(ms=ms, wall=wall, clocks=clk, launches=(l2 - l1), host=host, cost=cost, prof=eng.profile_dump() if profile else None,
+                    outputs=outputs)
 
     def rowstats(w, leg):
         """rows a step touches on this rank, and how many of them live on a peer (row % world != rank)"""
@@ -610,8 +649,11 @@ def main():
     # ------------------------------------------------------------------------------------------------ main line
     B = w["B"]
     eng = build_engine(w, B)
-    sharded = world > 1 and w["I"] * w["D"] * 4 > 32 * 2**20
-    leg = timed_leg(eng, w, B, args.steps, args.warmup)
+    leg = timed_leg(eng, w, B, args.steps, args.warmup, capture=bool(args.dump_outputs) and rank == 0)
+    if leg["outputs"] is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in leg["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     psteps = max(5, min(args.steps, 20))
     prof_leg = timed_leg(eng, w, B, psteps, 1, profile=True)
     rl, kern, nv = roofline_of(w, prof_leg, psteps, B, traffic_key=wname if world == 1 else None)
